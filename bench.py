@@ -25,6 +25,13 @@ Timing: W (>= 3) warm-up steps, then warm-up continues until 5 consecutive steps
 settled; at most ~3 s), then EXACTLY K steps between ``barrier + synchronize`` on both sides, one CUDA event per step
 (total = first → last event; median / p90 of the per-step times are reported too), max over ranks.  SM clocks and
 throttle reasons are read from NVML in-process (a 25 ms polling thread; no child process inside the timed region).
+
+``--dump-outputs DIR``: after everything above, the timed step runs once more and what it computed is written as
+``DIR/<name>.npy`` (``dump_outputs``), so that two builds run with the same arguments can be compared output for output.
+That step starts from the parameters and buffers the first training step started from, with a fresh optimizer, on the
+batch of the last timed step, so every run computes it from the same inputs.  The state at the end of the timed steps is
+not reproducible: each step leaves run-to-run rounding differences (BatchNorm statistics are summed with float atomics,
+cuDNN picks its algorithms by timing) and training amplifies them step after step.
 """
 from __future__ import annotations
 
@@ -62,7 +69,35 @@ def parse():
     ap.add_argument("--no-comparators", action="store_true", help="skip the same-invocation NCCL-PS / host comparators")
     ap.add_argument("--no-pipeline", action="store_true", help="one fused update launch inside step() (round-1 behaviour)")
     ap.add_argument("--profile", action="store_true", help="CUDA-event section timings of the PS path (stderr)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="afterwards, run the timed step once more from the start state on the last timed step's batch and "
+                         "write its loss, updated parameters and buffers as DIR/<name>.npy (float32)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, model, loss):
+    """``loss.npy`` (the step's loss), ``params.npy`` and ``buffers.npy`` (every parameter / floating-point buffer after the
+    step's update, flattened in logical order and concatenated in ``model.named_*`` order), all float32.  When they would
+    exceed ``DUMP_BYTES`` in all, ``params.npy`` holds the parameters at a fixed, seeded, sorted sample of positions."""
+    import numpy as np
+    with torch.no_grad():
+        params = torch.cat([p.detach().reshape(-1).float() for p in model.parameters()]).cpu()
+        bufs = [b.detach().reshape(-1).float() for b in model.buffers() if b.is_floating_point()]
+        bufs = torch.cat(bufs).cpu() if bufs else torch.zeros(0)
+        room = DUMP_BYTES // 4 - 1 - bufs.numel()
+        if params.numel() > room:
+            idx = torch.randint(0, params.numel(), (room,), generator=torch.Generator().manual_seed(0)).sort().values
+            params = params[idx]
+        arrays = {"loss": loss.detach().float().reshape(1).cpu(), "params": params, "buffers": bufs}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.numpy().astype(np.float32, copy=False))
 
 
 def reference_unavailable():
@@ -179,17 +214,29 @@ def main():
         return cls(named, [p for _, p in named], code=make_code(ps, args.code), mode=args.mode, engine="device",
                    average=True, profile=args.profile, pipeline=not args.no_pipeline, **hyper)
 
-    opt = make_opt("ours" if args.impl == "ours" else args.comparator_kind)
-    eng = getattr(opt, "_engine", None)
-    if args.bcast_gemm != "off" and eng is not None:
+    first_linear = []
+
+    def attach_gate(o):
+        """``--bcast-gemm``: bind the first forward GEMM to the device engine of optimizer ``o``."""
+        if args.bcast_gemm == "off" or getattr(o, "_engine", None) is None:
+            return
+        pull, gate = args.bcast_gemm == "pull", args.model == "mlp"
         if hasattr(model, "attach"):
-            model.attach(opt)                 # ResNet: the fused stem kernel acquires PARAMS_READY before its weight TMA
+            model.attach(o)                   # ResNet: the fused stem kernel acquires PARAMS_READY before its weight TMA
+        elif first_linear:
+            first_linear[0].attach(o, pull=pull, gate=gate)
         else:
             from pytorch_ps_mpi_b200.ops.linear import convert_first_linear
             # the in-kernel gate replaces the wait kernel only where the first linear is the first parameter consumer (MLP)
-            layer = convert_first_linear(model, opt, relu=(args.model == "mlp"), pull=(args.bcast_gemm == "pull"),
-                                         gate=(args.model == "mlp"))
+            layer = convert_first_linear(model, o, relu=(args.model == "mlp"), pull=pull, gate=gate)
             assert layer is not None, "model has no nn.Linear to convert"
+            first_linear.append(layer)
+
+    opt = make_opt("ours" if args.impl == "ours" else args.comparator_kind)
+    eng = getattr(opt, "_engine", None)
+    attach_gate(opt)
+    # --dump-outputs: the state the first training step starts from (every rank holds rank 0's weights by now)
+    start = {k: v.detach().clone() for k, v in model.state_dict().items()} if args.dump_outputs else None
 
     # distinct batches so no step re-reads a cached input; pinned host copies for the e2e arm
     gen = torch.Generator().manual_seed(1234 + w.rank)
@@ -418,6 +465,20 @@ def main():
         state["opt"] = None
     else:
         info = {"chunks": getattr(eng, "nchunks", None)}
+
+    # ---- --dump-outputs: the timed step once more, from the saved start state, on the last timed step's batch ----
+    if args.dump_outputs:
+        if state["opt"] is not None:
+            state["opt"].close()
+        if hasattr(model, "attach"):
+            model._engine = None              # the gate belonged to the engine that was just closed
+        model.load_state_dict(start)
+        state["opt"] = make_opt("ours" if args.impl == "ours" else args.comparator_kind)
+        attach_gate(state["opt"])
+        loss = train_step(*dev[(K - 1) % nbuf])
+        torch.cuda.synchronize(device)
+        if w.rank == 0:                       # rank 0 holds the server's parameters
+            dump_outputs(args.dump_outputs, model, loss)
 
     if w.rank == 0:
         out = {

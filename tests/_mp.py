@@ -4,6 +4,10 @@ import os
 import numpy as np
 import torch
 
+#: environment of the ranks of the CPU scenarios: no visible GPU, so ``runtime.init()`` builds a CPU / gloo world on any
+#: machine (with a GPU visible every rank would pick ``cuda:0`` and NCCL, which refuses two ranks on one device)
+CPU_ONLY = {"CUDA_VISIBLE_DEVICES": ""}
+
 
 def _world(rank, size):
     import pytorch_ps_mpi_b200 as ps

@@ -203,6 +203,36 @@ def test_bench_with_same_invocation_comparators(bench_env, monkeypatch, capsys):
     assert all(k in out["comparators"] and "value" in out["comparators"][k] for k in (out["vs_comparator"] or {}))
 
 
+def test_bench_dump_outputs_do_not_depend_on_the_timed_steps(bench_env, monkeypatch, capsys, tmp_path):
+    """``--dump-outputs``: the timed step once more, from the start state, on the last timed step's batch; its loss, parameters
+    and buffers as float32 ``.npy`` files.  Runs whose last timed batch is the same (2 and 6 steps over 4 rotating batches) write
+    the same arrays, whatever the timed, warm-up and comparator steps did before (the emulated kernels are deterministic)."""
+    import numpy as np
+    bench, extm = bench_env
+    runs = []
+    for k, (steps, extra) in enumerate(((2, ["--no-comparators"]), (6, []))):       # the second run also trains the comparators
+        d = tmp_path / str(k)
+        out = _run_bench(bench, extm, 1, ["--steps", str(steps), "--warmup", "3", "--batch", "2", "--no-e2e",
+                                          "--dump-outputs", str(d)] + extra, monkeypatch, capsys)
+        assert out["steps"] == steps
+        runs.append({name: np.load(d / f"{name}.npy") for name in ("loss", "params", "buffers")})
+    model = MI._tiny_resnet()
+    assert runs[0]["loss"].shape == (1,)
+    assert runs[0]["params"].shape == (sum(p.numel() for p in model.parameters()),)
+    assert runs[0]["buffers"].shape == (sum(b.numel() for b in model.buffers() if b.is_floating_point()),)
+    for name, a in runs[0].items():
+        assert a.dtype == np.float32 and np.isfinite(a).all(), name
+        np.testing.assert_array_equal(a, runs[1][name], err_msg=name)
+    assert not np.array_equal(runs[0]["params"], torch.cat([p.detach().reshape(-1).float() for p in model.parameters()]).numpy())
+
+
+def test_bench_rejects_fewer_than_one_step(monkeypatch):
+    import bench
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "0"])
+    with pytest.raises(SystemExit):
+        bench.parse()
+
+
 def test_bench_reference_arm_reports_unavailable(monkeypatch, capsys):
     import bench
     monkeypatch.setattr(sys, "argv", ["bench.py", "--impl", "reference", "--gpus", "1"])

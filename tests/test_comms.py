@@ -19,7 +19,7 @@ def test_gather_bcast_iallgather_any_source(transport, n):
     """The reference's three test files re-created (``test_comms.py:9-26``, ``test_iallgather.py:37-54``, ``test_mpi.py:34-96``)
     + any-source point-to-point, at 2 and 3 ranks over both transports — one set of processes per (transport, n)."""
     names = ["gather_objects", "bcast_objects"] + (["iallgather_objects", "p2p_any_source"] if n == 3 else [])
-    spawn(_mp.comm_suite, n, (transport, names), timeout=240)
+    spawn(_mp.comm_suite, n, (transport, names), env=_mp.CPU_ONLY, timeout=240)
 
 
 def test_single_process_world():
@@ -39,4 +39,4 @@ def test_single_process_world():
 
 def test_shm_transport_stress():
     """Native ShmComm under load: 4 ranks, 64 KB rings, up to 300 KB messages, 30 rounds of all-to-all."""
-    spawn(_mp.shm_stress, 4, timeout=240)
+    spawn(_mp.shm_stress, 4, env=_mp.CPU_ONLY, timeout=240)

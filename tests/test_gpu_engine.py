@@ -248,10 +248,13 @@ def test_direct_gradient_placement_matches_encode_path(monkeypatch):
     assert nb == 0 and na >= 41, (na, nb)          # 20 BN layers x (gamma, beta) + the stem weight
     # BatchNorm statistics are summed with float atomics, so two runs of the SAME path already differ in the last bits and a
     # randomly initialised ResNet at batch 8 amplifies that: the encode path must agree with the direct path as well as the
-    # direct path agrees with itself
+    # direct path agrees with itself.  Such a last-bit difference can flip the rounding of a bf16 parameter by one step even
+    # where the two direct runs happened to round alike, so the floor is one bf16 step of the value (and at least 2e-3)
+    half_eps = torch.finfo(torch.bfloat16).eps / 2
     for p, p2, q in zip(a, a2, b):
         noise = float((p - p2).abs().max())
-        assert float((p - q).abs().max()) <= 8.0 * noise + 2e-3, (float((p - q).abs().max()), noise)
+        bf16_step = torch.ldexp(torch.full_like(p, half_eps), torch.frexp(p).exponent) * (p != 0)
+        assert bool(((p - q).abs() <= 8.0 * noise + bf16_step.clamp(min=2e-3)).all()), (float((p - q).abs().max()), noise)
 
 
 def test_stem_weight_lives_in_gemm_layout_in_the_arena():

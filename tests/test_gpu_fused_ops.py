@@ -52,7 +52,7 @@ def test_implicit_stem_wgrad(shape):
     assert _rel(stem_wgrad_implicit(x, g), ref) < 1e-2
 
 
-def test_fused_stem_autograd_matches_default_path():
+def test_fused_stem_autograd_matches_default_path(monkeypatch):
     from pytorch_ps_mpi_b200.ops import stem as stem_mod
     dev = torch.device("cuda", 0)
     torch.manual_seed(0)
@@ -61,12 +61,11 @@ def test_fused_stem_autograd_matches_default_path():
     gy = _cl(torch.randn(4, 64, 112, 112, device=dev).bfloat16())
     grads = []
     for fused, implicit in ((False, False), (True, False), (True, True)):
-        stem_mod._IMPLICIT_WGRAD = implicit
+        monkeypatch.setattr(stem_mod, "_IMPLICIT_WGRAD", implicit)       # restored after the test: later tests see the default
         wv = wt.clone().requires_grad_(True)
         y = stem_mod.stem_conv_fused(x, wv)[0] if fused else stem_mod.stem_conv(x, wv)
         y.backward(gy)
         grads.append(wv.grad.float())
-    stem_mod._IMPLICIT_WGRAD = False
     assert _rel(grads[1], grads[0]) < 1e-2 and _rel(grads[2], grads[0]) < 1e-2
 
 

@@ -21,27 +21,27 @@ SYNC_CASES = {          # (mode, optim, coding, coalesce)
 @pytest.mark.parametrize("transport", ["shm", "gloo"])
 def test_mlp_sync(transport):
     """Every scenario of a transport runs in one pair of processes (see ``_mp.mlp_train_many``)."""
-    spawn(_mp.mlp_train_many, 2, (transport, SYNC_CASES[transport]), timeout=300)
+    spawn(_mp.mlp_train_many, 2, (transport, SYNC_CASES[transport]), env=_mp.CPU_ONLY, timeout=300)
 
 
 @pytest.mark.parametrize("transport", ["shm", "gloo"])
 def test_three_ranks_sync_average_groups_async(transport):
     """3 ranks: sync PS vs the oracle (shm), ``average=True`` + several param groups, AsySG-InCon with quota 1 (both transports)."""
-    spawn(_mp.three_rank_suite, 3, (transport,), timeout=300)
+    spawn(_mp.three_rank_suite, 3, (transport,), env=_mp.CPU_ONLY, timeout=300)
 
 
 def test_shm_transport_detects_dead_peer():
     from pytorch_ps_mpi_b200.launch import spawn as _spawn
     import multiprocessing
     # rank 1 exits with os._exit(0) on purpose; rank 0 must notice instead of hanging
-    _spawn(_mp.shm_dead_peer, 2, timeout=90)
+    _spawn(_mp.shm_dead_peer, 2, env=_mp.CPU_ONLY, timeout=90)
 
 
 def test_async_consistent_reads():
-    spawn(_mp.mlp_async_consistent, 3)
+    spawn(_mp.mlp_async_consistent, 3, env=_mp.CPU_ONLY)
 
 
 @pytest.mark.parametrize("n", [2, 3])
 def test_reference_equivalent_comparator(n):
     """The comparator bench.py runs in the same invocation as the product arm: right numerics, no hang, on gloo."""
-    spawn(_mp.comparator_host, n, env={"PSB200_TRANSPORT": "gloo"}, timeout=180)
+    spawn(_mp.comparator_host, n, env=dict(_mp.CPU_ONLY, PSB200_TRANSPORT="gloo"), timeout=180)
