@@ -84,12 +84,27 @@ def peer_copy_gbs(w, dev, nbytes=256 << 20):
     return out
 
 
+def sweep_code(name):
+    kind, _, arg = name.partition(":")
+    if kind == "identity":
+        return ps.Identity()
+    if kind == "topk":
+        return ps.TopK(ratio=float(arg), values="bf16")
+    if kind == "cast":
+        return ps.Cast(arg)
+    if kind == "scale":
+        return ps.Scale(arg or "int8")
+    if kind == "qsgd":
+        return ps.QSGD(levels=int(arg or 127), blockwise=True, seed=0)
+    raise ValueError(f"unknown --code {name!r}")
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--min-kb", type=float, default=1)
     ap.add_argument("--max-mb", type=float, default=256)
     ap.add_argument("--dtype", default="bf16")
-    ap.add_argument("--code", default="identity")
+    ap.add_argument("--code", default="identity", help="identity | cast:DT | scale:DT | topk:RATIO | qsgd:LEVELS")
     ap.add_argument("--impls", default="fused,nccl,host")
     ap.add_argument("--reduce", default="auto")
     ap.add_argument("--piece-mb", type=float, default=8.0, help="largest tensor of the synthetic parameter vector")
@@ -126,9 +141,7 @@ def main():
             opt = eng = None
             wire = n * esz
             if impl == "fused":
-                code = ps.Identity() if a.code == "identity" else (
-                    ps.TopK(ratio=float(a.code.split(":")[1]), values="bf16") if a.code.startswith("topk") else
-                    ps.Cast(a.code.split(":")[1]))
+                code = sweep_code(a.code)
                 named = [(f"v{i}", p) for i, p in enumerate(params)]
                 opt = ps.SGD(named, params, lr=1e-3, code=code, mode="ps", engine="device", reduce=a.reduce, cuda=True)
                 eng = opt._engine

@@ -9,7 +9,8 @@ uses exactly three members of the object passed as ``code=``:
   decoding (``ps.py:165``).
 
 This module ships that contract as :class:`Coding` plus the built-ins the framework fuses into
-its sm_100a kernels: :class:`Identity`, :class:`Cast`, :class:`Scale`, :class:`TopK`.  Each
+its sm_100a kernels: :class:`Identity`, :class:`Cast`, :class:`Scale`, :class:`TopK` and block-wise
+:class:`QSGD`.  Each
 built-in has
 
 * a pure-PyTorch ``encode``/``decode`` (host slow path **and** the numerical oracle every CUDA
@@ -21,6 +22,7 @@ Arbitrary user codings (any object with ``encode``/``decode``) keep working on t
 """
 from __future__ import annotations
 
+import itertools
 import math
 from dataclasses import dataclass
 from typing import Any, List, Optional
@@ -30,7 +32,8 @@ import torch
 __all__ = [
     "Coding", "Identity", "Cast", "Scale", "TopK", "QSGD", "SVD", "DeviceCodeSpec", "TILE",
     "WIRE_F32", "WIRE_BF16", "WIRE_F16", "WIRE_E4M3", "WIRE_E5M2", "WIRE_I8",
-    "KIND_DENSE", "KIND_SCALED", "KIND_TOPK", "wire_dtype_of", "wire_code_of", "tile_k",
+    "KIND_DENSE", "KIND_SCALED", "KIND_TOPK", "KIND_QSGD", "wire_dtype_of", "wire_code_of", "tile_k",
+    "qsgd_uniform16", "qsgd_blockwise",
 ]
 
 #: elements per tile of the flat arena; every parameter starts on a tile boundary and the
@@ -40,7 +43,7 @@ TILE = 2048
 # wire element types (must match csrc/kernels/common.cuh)
 WIRE_F32, WIRE_BF16, WIRE_F16, WIRE_E4M3, WIRE_E5M2, WIRE_I8 = 0, 1, 2, 3, 4, 5
 # coding kinds
-KIND_DENSE, KIND_SCALED, KIND_TOPK = 0, 1, 2
+KIND_DENSE, KIND_SCALED, KIND_TOPK, KIND_QSGD = 0, 1, 2, 3
 
 _WIRE_TORCH = {
     WIRE_F32: torch.float32, WIRE_BF16: torch.bfloat16, WIRE_F16: torch.float16,
@@ -82,10 +85,12 @@ def tile_k(ratio: float, valid: int) -> int:
 class DeviceCodeSpec:
     """Fixed binary wire layout of a built-in coding (consumed by the CUDA kernels)."""
 
-    kind: int                 # KIND_DENSE | KIND_SCALED | KIND_TOPK
+    kind: int                 # KIND_DENSE | KIND_SCALED | KIND_TOPK | KIND_QSGD
     wire: int                 # WIRE_* element type of the payload values (-1 = same as grad)
     ratio: float = 1.0        # top-k keep ratio (KIND_TOPK)
     error_feedback: bool = False
+    levels: int = 0           # quantisation levels (KIND_QSGD)
+    seed: int = 0             # 64-bit Philox key (KIND_QSGD)
 
     def resolved_wire(self, grad_dtype: torch.dtype) -> int:
         return wire_code_of(grad_dtype) if self.wire < 0 else self.wire
@@ -101,6 +106,8 @@ class DeviceCodeSpec:
             # entry = value + index packed to 2x the value width (bf16+u16 / f32+u32)
             esz = 4 if esz <= 2 else 8
             n = self.tile_capacity() * esz
+        elif self.kind == KIND_QSGD:
+            n = TILE * esz + 4            # int8 payload + the tile's fp32 scale (trailer zero-padded to 16 bytes)
         else:
             n = TILE * esz
         return (n + 15) // 16 * 16
@@ -323,20 +330,141 @@ class TopK(Coding):
         return f"TopK({what}, values={_WIRE_TORCH[self.wire]}, exact={self.exact})"
 
 
+_PHILOX_M0, _PHILOX_M1, _PHILOX_W0, _PHILOX_W1 = 0xD2511F53, 0xCD9E8D57, 0x9E3779B9, 0xBB67AE85
+_U32 = 0xFFFFFFFF
+
+
+def _mulhilo32(a: int, b: torch.Tensor):
+    """``(hi, lo)`` 32-bit halves of the 64-bit product of the constant ``a`` and int64 tensor ``b`` (values < 2**32), in
+    int64 arithmetic that never overflows: ``a`` is split into 16-bit halves."""
+    t_lo, t_hi = b * (a & 0xFFFF), b * (a >> 16)          # each < 2**48
+    s = t_lo + ((t_hi & 0xFFFF) << 16)                     # < 2**49
+    return (t_hi >> 16) + (s >> 32), s & _U32
+
+
+def qsgd_uniform16(seed: int, rank: int, step: int, first_elem: int, n: int, device=None) -> torch.Tensor:
+    """The 16-bit uniforms the block-wise QSGD kernel draws for arena elements ``[first_elem, first_elem + n)`` (int32 tensor).
+
+    Philox4x32-10 with the Random123 constants, one call per 8 consecutive elements ``e0 .. e0 + 7`` (``e0 % 8 == 0``):
+    counter = ``(e0 / 8 low 32 bits, e0 / 8 high 32 bits, step, rank)``, key = ``(seed low 32 bits, seed high 32 bits)``;
+    element ``e0 + j`` takes 16 bits of output word ``j >> 1`` (low half for even ``j``).  Runs on ``device`` in int64 ops."""
+    g0 = int(first_elem) // 8
+    k = torch.arange((int(first_elem) + n + 7) // 8 - g0, dtype=torch.int64, device=device)
+    lo = (g0 & _U32) + k                                   # the 64-bit group index as two words (any index, no int64 overflow)
+    c0, c1 = lo & _U32, ((g0 >> 32) + (lo >> 32)) & _U32
+    c2 = torch.full_like(c0, int(step) & _U32)
+    c3 = torch.full_like(c0, int(rank) & _U32)
+    k0, k1 = int(seed) & _U32, (int(seed) >> 32) & _U32
+    for _ in range(10):
+        hi0, lo0 = _mulhilo32(_PHILOX_M0, c0)
+        hi1, lo1 = _mulhilo32(_PHILOX_M1, c2)
+        c0, c1, c2, c3 = hi1 ^ c1 ^ k0, lo1, hi0 ^ c3 ^ k1, lo0
+        k0, k1 = (k0 + _PHILOX_W0) & _U32, (k1 + _PHILOX_W1) & _U32
+    words = torch.stack([c0, c1, c2, c3], dim=1)                              # [groups, 4]
+    u = torch.stack([words & 0xFFFF, words >> 16], dim=2).reshape(-1)       # [groups * 8] in element order
+    off = int(first_elem) - 8 * g0
+    return u[off: off + n].to(torch.int32)
+
+
+def qsgd_blockwise(flat: torch.Tensor, levels: int, u16: torch.Tensor):
+    """Block-wise QSGD of a flat tensor with the given 16-bit uniforms: ``(q int8 [ntiles * TILE], scale fp32 [ntiles])``.
+
+    The bit-exact oracle of the ``KIND_QSGD`` encode kernel.  Per ``TILE``-element tile: ``norm = sqrt(sum of squares)``
+    summed in the kernel's order (a thread's 8 elements in sequence, an xor butterfly over the 32 lanes of a warp, then the 8
+    warp sums in order), ``x = min(|g| * (levels / norm), levels)``, ``q = sign(g) * (floor(x) + [u16 < frac(x) * 2**16])``
+    and ``scale = norm / levels``.  A tile whose norm is zero or not finite gets ``q = 0`` and ``scale = 0``."""
+    g = flat.reshape(-1).float()
+    n = g.numel()
+    nt = max(1, -(-n // TILE))
+    pad = nt * TILE - n
+    u = u16.reshape(-1)[: nt * TILE]
+    if pad:
+        g = torch.cat([g, g.new_zeros(pad)])
+    if u.numel() < nt * TILE:
+        u = torch.cat([u, u.new_zeros(nt * TILE - u.numel())])
+    sq = (g * g).view(nt, TILE // 8, 8)
+    s = sq[:, :, 0]
+    for j in range(1, 8):
+        s = s + sq[:, :, j]
+    s = s.reshape(nt, TILE // 256, 32)
+    lanes = torch.arange(32, device=g.device)
+    for off in (16, 8, 4, 2, 1):
+        s = s + s[:, :, lanes ^ off]
+    tot = s[:, 0, 0]
+    for w in range(1, TILE // 256):
+        tot = tot + s[:, w, 0]
+    norm = _sqrt_rn(tot)
+    live = (norm > 0) & torch.isfinite(norm)
+    lv = torch.full_like(norm, float(levels))
+    r = lv / norm                                   # tensor / tensor: IEEE division on every device
+    x = torch.minimum(g.view(nt, TILE).abs() * r[:, None], lv[:, None])
+    low = torch.floor(x)
+    up = u.view(nt, TILE).float() < (x - low) * 65536.0
+    q = torch.copysign(low + up.float(), g.view(nt, TILE))
+    q = torch.where(live[:, None], q, torch.zeros_like(q))
+    scale = torch.where(live, norm / lv, torch.zeros_like(norm))
+    return q.to(torch.int8).reshape(-1), scale
+
+
+def _sqrt_rn(x: torch.Tensor) -> torch.Tensor:
+    """Correctly rounded fp32 square root (``__fsqrt_rn``) on any device: torch's vectorised CPU ``sqrt`` is not.  A
+    neighbour of ``r`` is taken when the exact square of the midpoint between them (25-bit operands, exact in fp64) lies on
+    the other side of ``x``."""
+    r = torch.sqrt(x.double()).float()
+    xd = x.double()
+    for _ in range(2):
+        up, dn = torch.nextafter(r, torch.full_like(r, math.inf)), torch.nextafter(r, torch.zeros_like(r))
+        r = torch.where(((r.double() + up.double()) / 2) ** 2 < xd, up, r)
+        r = torch.where(((r.double() + dn.double()) / 2) ** 2 > xd, dn, r)
+    return r
+
+
+def _host_rank() -> int:
+    from . import runtime
+    return runtime.world().rank if runtime.is_initialized() else 0
+
+
 class QSGD(Coding):
     """QSGD-style stochastic quantisation (Alistarh et al. 2017): ``sign · ‖g‖₂ · ξ/levels`` with ``ξ`` drawn so
-    the code is an unbiased estimate of the gradient.  Host (generic-object) path — the kind of user coding the
-    reference's external ``codings`` module carried (SURVEY §2.2); the fused device codings are
-    :class:`Cast` / :class:`Scale` / :class:`TopK`.
+    the code is an unbiased estimate of the gradient.
+
+    * ``blockwise=False`` (default): one norm per tensor, ``torch.rand`` rounding.  Host (generic-object) path — the kind of
+      user coding the reference's external ``codings`` module carried (SURVEY §2.2).
+    * ``blockwise=True``: one norm per ``TILE``-element tile of the flat arena ("bucketed" QSGD with bucket size ``TILE``),
+      ``1 <= levels <= 127`` on an int8 wire.  Fused on device (``KIND_QSGD``): each tile travels as ``TILE`` int8 codes plus
+      its fp32 ``scale = norm / levels``; there is no abs-max pre-pass and no size exchange.  The rounding draws come from
+      Philox4x32-10 keyed by ``(seed, rank, step, arena element)`` (:func:`qsgd_uniform16`), so a seeded run is reproducible.
+      A draw has 16 bits, which biases each rounding by at most 2⁻¹⁶ of one quantum (``scale``); otherwise
+      ``E[decode(encode(g))] = g``.  ``seed=None`` draws a 64-bit seed once, here, from torch's global CPU generator; ranks
+      need not agree on it because the rank is part of the Philox counter.  The host ``encode`` runs the same per-tile
+      algorithm on the gradient's own device (``rank`` / ``step`` / ``first_elem`` default to this process's rank, a
+      per-instance call counter and 0).
     """
 
-    def __init__(self, levels: int = 255, seed: Optional[int] = None):
+    def __init__(self, levels: int = 255, seed: Optional[int] = None, blockwise: bool = False):
         if not 1 <= levels <= 32767:
             raise ValueError("levels must be in [1, 32767]")
         self.levels = int(levels)
-        self._gen = torch.Generator().manual_seed(seed) if seed is not None else None
+        self.blockwise = bool(blockwise)
+        if self.blockwise:
+            if self.levels > 127:
+                raise ValueError("QSGD(blockwise=True) needs 1 <= levels <= 127 (the wire is int8)")
+            if seed is None:
+                lo, hi = torch.randint(0, 1 << 32, (2,), dtype=torch.int64).tolist()
+                seed = lo | hi << 32
+            self.seed = int(seed) & ((1 << 64) - 1)
+            self._calls = itertools.count()
+        else:
+            self._gen = torch.Generator().manual_seed(seed) if seed is not None else None
 
-    def encode(self, grad, **kwargs):
+    def encode(self, grad, rank=None, step=None, first_elem=0, **kwargs):
+        if self.blockwise:
+            g = grad.detach()
+            rank = _host_rank() if rank is None else rank
+            step = next(self._calls) if step is None else step
+            u = qsgd_uniform16(self.seed, rank, step, first_elem, g.numel(), device=g.device)
+            q, scale = qsgd_blockwise(g, self.levels, u)
+            return {"q": q, "scale": scale, "shape": tuple(g.shape)}
         g = grad.detach().float().cpu()
         norm = g.norm()
         if float(norm) == 0.0 or not torch.isfinite(norm):
@@ -350,12 +478,22 @@ class QSGD(Coding):
         return {"q": q.to(dt), "norm": norm.reshape(1), "levels": self.levels, "shape": tuple(g.shape)}
 
     def decode(self, code, cuda=False):
+        shape = tuple(int(d) for d in code["shape"])
+        if "scale" in code:                                   # block-wise: one scale per tile
+            q = self._place(_as_tensor(code["q"]), cuda).float()
+            scale = self._place(_as_tensor(code["scale"]), cuda).float()
+            return (q.view(-1, TILE) * scale[:, None]).reshape(-1)[: math.prod(shape)].reshape(shape)
         q = self._place(_as_tensor(code["q"]), cuda).float()
         norm = self._place(_as_tensor(code["norm"]), cuda).float()
-        return (q * (norm / float(code["levels"]))).reshape(tuple(int(d) for d in code["shape"]))
+        return (q * (norm / float(code["levels"]))).reshape(shape)
+
+    def device_spec(self):
+        if not self.blockwise:
+            return None
+        return DeviceCodeSpec(KIND_QSGD, WIRE_I8, levels=self.levels, seed=self.seed)
 
     def __repr__(self):
-        return f"QSGD(levels={self.levels})"
+        return f"QSGD(levels={self.levels}, blockwise=True)" if self.blockwise else f"QSGD(levels={self.levels})"
 
 
 class SVD(Coding):

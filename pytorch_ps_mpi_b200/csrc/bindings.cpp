@@ -125,7 +125,7 @@ void encode(int kind, int wire, const std::vector<at::Tensor>& grads, const std:
             const std::vector<int>& ntiles, const std::vector<int>& param_idx, uint64_t tiles_ptr, uint64_t wire_ptr,
             uint64_t scales_ptr, uint64_t amax_ptr, uint64_t residual_ptr, int bytes_per_tile, int cap, double ratio,
             const std::vector<uint64_t>& sig_targets, int sig_slot, uint64_t sig_value, uint64_t sig_counter,
-            uint64_t stream) {
+            uint64_t stream, int levels, uint64_t seed, uint32_t rng_step, int rank) {
   const size_t n = grads.size();
   if (first_tile.size() != n || ntiles.size() != n || param_idx.size() != n) throw std::runtime_error("encode: length mismatch");
   if (n == 0) return;
@@ -140,6 +140,14 @@ void encode(int kind, int wire, const std::vector<at::Tensor>& grads, const std:
   a.cap = cap;
   a.ratio = ratio;
   a.grad_dt = dt_code(grads[0].scalar_type());
+  if (kind == KIND_QSGD) {
+    if (levels < 1 || levels > 127) throw std::runtime_error("encode: QSGD levels must be in [1, 127] (int8 wire)");
+    if (bytes_per_tile < PSB_TILE + 16) throw std::runtime_error("encode: a QSGD wire slot needs TILE + 16 bytes");
+  }
+  a.levels = levels;
+  a.seed = seed;
+  a.rng_step = rng_step;
+  a.rank = rank;
   for (size_t base = 0; base < n; base += PSB_ENCODE_MAX) {
     const int m = (int)std::min<size_t>(PSB_ENCODE_MAX, n - base);
     a.batch.n = m;
@@ -290,7 +298,8 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
         py::arg("param_idx"), py::arg("tiles_ptr"), py::arg("wire_ptr"), py::arg("scales_ptr"), py::arg("amax_ptr"),
         py::arg("residual_ptr"), py::arg("bytes_per_tile"), py::arg("cap"), py::arg("ratio"),
         py::arg("sig_targets") = std::vector<uint64_t>{}, py::arg("sig_slot") = 0, py::arg("sig_value") = 0,
-        py::arg("sig_counter") = 0, py::arg("stream") = 0);
+        py::arg("sig_counter") = 0, py::arg("stream") = 0, py::arg("levels") = 0, py::arg("seed") = 0, py::arg("rng_step") = 0,
+        py::arg("rank") = 0);
   m.def("signal", &signal, py::arg("targets"), py::arg("slot"), py::arg("value"), py::arg("extra_slot") = -1,
         py::arg("extra_value") = 0, py::arg("stream") = 0, py::arg("version_local") = 0, py::arg("version_slot") = 0);
   m.def("wait_flags", &wait_flags, py::arg("signal_local"), py::arg("slot0"), py::arg("mask"), py::arg("want"),

@@ -23,7 +23,7 @@
 // wire element types (codings.py WIRE_*)
 enum : int { WIRE_F32 = 0, WIRE_BF16 = 1, WIRE_F16 = 2, WIRE_E4M3 = 3, WIRE_E5M2 = 4, WIRE_I8 = 5 };
 // coding kinds (codings.py KIND_*)
-enum : int { KIND_DENSE = 0, KIND_SCALED = 1, KIND_TOPK = 2 };
+enum : int { KIND_DENSE = 0, KIND_SCALED = 1, KIND_TOPK = 2, KIND_QSGD = 3 };
 // parameter / gradient dtypes
 enum : int { DT_F32 = 0, DT_BF16 = 1, DT_F16 = 2 };
 // optimizers

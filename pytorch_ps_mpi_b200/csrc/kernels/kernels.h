@@ -27,6 +27,11 @@ struct EncodeArgs {
   int32_t cap;           // top-k entries per tile
   double ratio;
   int32_t grad_dt;
+  // block-wise QSGD (KIND_QSGD): quantisation levels and the Philox key / counter words of this launch
+  int32_t levels;
+  uint64_t seed;
+  uint32_t rng_step;
+  int32_t rank;
   // optional fused flag raise: when this is the LAST encode launch of the step, its last CTA publishes
   // GRAD_READY itself (saves the separate psb_signal_kernel launch on the critical path)
   uint64_t* sig_targets[PSB_MAX_RANKS];

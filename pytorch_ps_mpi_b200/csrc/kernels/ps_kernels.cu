@@ -80,6 +80,29 @@ __device__ __forceinline__ void load_grad8(const EncodeArgs& a, int entry, const
   }
 }
 
+// A product rounded on its own, which the compiler may not fuse with a following add into an FMA: the QSGD tile norm is
+// specified operation by operation (codings.qsgd_blockwise reproduces it).  Compiled as plain host C++, as the CPU
+// emulator does, there is no FMA to fuse into.
+#ifdef __CUDACC__
+__device__ __forceinline__ float mul_rn(float a, float b) { return __fmul_rn(a, b); }
+#else
+inline float mul_rn(float a, float b) { return a * b; }
+#endif
+
+// Philox4x32-10 (Salmon et al., SC'11; Random123 constants).  The mul-hi is the top half of a 64-bit product so that the
+// same text runs in the CPU emulator; codings.qsgd_uniform16 is the Python mirror.
+__device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1,
+                                              uint32_t* out) {
+#pragma unroll
+  for (int i = 0; i < 10; ++i) {
+    const uint64_t p0 = (uint64_t)0xD2511F53u * c0, p1 = (uint64_t)0xCD9E8D57u * c2;
+    const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c1 ^ k0, n2 = (uint32_t)(p0 >> 32) ^ c3 ^ k1;
+    c0 = n0, c1 = (uint32_t)p1, c2 = n2, c3 = (uint32_t)p0;
+    k0 += 0x9E3779B9u, k1 += 0xBB67AE85u;
+  }
+  out[0] = c0, out[1] = c1, out[2] = c2, out[3] = c3;
+}
+
 // ------------------------------------------------------------------------------------------
 // abs-max pre-pass for Scale codings: one atomicMax per tile into amax_bits[param]
 // ------------------------------------------------------------------------------------------
@@ -98,7 +121,7 @@ __global__ void __launch_bounds__(PSB_THREADS) psb_absmax_kernel(const __grid_co
 }
 
 // ------------------------------------------------------------------------------------------
-// encode: gradient tile → wire tile (dense cast | abs-max scaled | block-wise top-k)
+// encode: gradient tile → wire tile (dense cast | abs-max scaled | block-wise top-k | block-wise QSGD)
 // ------------------------------------------------------------------------------------------
 template <int WIRE>
 __device__ __forceinline__ void store_dense(void* wire_tile, const float* q) {
@@ -144,6 +167,48 @@ __global__ void __launch_bounds__(PSB_THREADS) psb_encode_kernel(const __grid_co
 #pragma unroll
     for (int j = 0; j < PSB_EPT; ++j) q[j] = __fdiv_rn(g[j], inv);
     store_dense<WIRE>(wire_tile, q);
+  } else if constexpr (KIND == KIND_QSGD) {
+    // block-wise QSGD: q = sign(g) * stochastic_round(|g| * levels / ||tile||), scale = ||tile|| / levels in the slot trailer.
+    // The sum of squares runs in a fixed order that codings.qsgd_blockwise reproduces bit for bit: each thread's 8 elements in
+    // sequence, an xor butterfly over lanes (offsets 16..1), then the 8 warp sums in index order; the squares are not fused
+    // into the sum (mul_rn).  The rest is adds, subtractions and products that have no FMA form.
+    __shared__ float s_warp[PSB_THREADS / 32];
+    float ss = 0.f;
+#pragma unroll
+    for (int j = 0; j < PSB_EPT; ++j) ss += mul_rn(g[j], g[j]);
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, off);
+    if ((tid & 31) == 0) s_warp[tid >> 5] = ss;
+    __syncthreads();
+    float sum = s_warp[0];
+#pragma unroll
+    for (int w = 1; w < PSB_THREADS / 32; ++w) sum += s_warp[w];
+    const float norm = __fsqrt_rn(sum);
+    const float lv = (float)a.levels;
+    const bool live = norm > 0.f && isfinite(norm);     // an all-zero or non-finite tile travels as q = 0, scale = 0
+    float q[PSB_EPT];
+    if (live) {
+      // one Philox call per thread: counter = (arena element / 8, step, rank), key = seed → 8 uniforms of 16 bits
+      const uint64_t grp = ((uint64_t)tile * PSB_TILE + tid * PSB_EPT) / PSB_EPT;
+      uint32_t u[4];
+      philox4x32_10((uint32_t)grp, (uint32_t)(grp >> 32), a.rng_step, (uint32_t)a.rank, (uint32_t)a.seed,
+                    (uint32_t)(a.seed >> 32), u);
+      const float r = __fdiv_rn(lv, norm);
+#pragma unroll
+      for (int j = 0; j < PSB_EPT; ++j) {
+        const float x = fminf(fabsf(g[j]) * r, lv);   // rounding can land one ulp above `levels`: clamp
+        const float l = floorf(x);
+        const float u16 = (float)((u[j >> 1] >> (16 * (j & 1))) & 0xffffu);
+        const float up = u16 < (x - l) * 65536.f ? 1.f : 0.f;
+        q[j] = copysignf(l + up, g[j]);
+      }
+    } else {
+#pragma unroll
+      for (int j = 0; j < PSB_EPT; ++j) q[j] = 0.f;
+    }
+    store_dense<WIRE>(wire_tile, q);
+    if (tid == 0)
+      st_v4(wire_tile + PSB_TILE, make_uint4(__float_as_uint(live ? __fdiv_rn(norm, lv) : 0.f), 0u, 0u, 0u));
   } else {  // KIND_TOPK: block-wise magnitude top-k, ties → lower index, entries in index order
     __shared__ uint32_t hist[256];
     __shared__ uint32_t warp_tot[PSB_THREADS / 32];
@@ -569,6 +634,9 @@ __global__ void __launch_bounds__(PSB_THREADS, 3) psb_update_kernel(const __grid
             if (r < a.world && (contrib >> r & 1u)) {
               issue_dense<WIRE>(a.wire[r], (size_t)tile * a.bytes_per_tile, v0[c], v1[c]);
               if constexpr (KIND == KIND_SCALED) sc[c] = ld_sys_f32(a.scales[r] + ti.param);
+              if constexpr (KIND == KIND_QSGD)      // the tile's own scale, in the trailer of its wire slot
+                sc[c] = ld_sys_f32(reinterpret_cast<const float*>(reinterpret_cast<const uint8_t*>(a.wire[r]) +
+                                                                  (size_t)tile * a.bytes_per_tile + PSB_TILE));
             }
           }
 #pragma unroll
@@ -579,7 +647,7 @@ __global__ void __launch_bounds__(PSB_THREADS, 3) psb_update_kernel(const __grid
               decode_dense<WIRE>(v0[c], v1[c], f);
 #pragma unroll
               for (int j = 0; j < PSB_EPT; ++j) {
-                if constexpr (KIND == KIND_SCALED) acc[j] += f[j] * sc[c];
+                if constexpr (KIND == KIND_SCALED || KIND == KIND_QSGD) acc[j] += f[j] * sc[c];
                 else acc[j] += f[j];
               }
             }
@@ -847,7 +915,7 @@ void psb_launch_encode(cudaStream_t s, int kind, int wire, const EncodeArgs& a) 
   }
   ENC(KIND_DENSE, WIRE_F32) ENC(KIND_DENSE, WIRE_BF16) ENC(KIND_DENSE, WIRE_F16) ENC(KIND_DENSE, WIRE_E4M3)
   ENC(KIND_DENSE, WIRE_E5M2) ENC(KIND_SCALED, WIRE_I8) ENC(KIND_SCALED, WIRE_E4M3) ENC(KIND_SCALED, WIRE_E5M2)
-  ENC(KIND_SCALED, WIRE_F16) ENC(KIND_TOPK, WIRE_F32) ENC(KIND_TOPK, WIRE_BF16)
+  ENC(KIND_SCALED, WIRE_F16) ENC(KIND_TOPK, WIRE_F32) ENC(KIND_TOPK, WIRE_BF16) ENC(KIND_QSGD, WIRE_I8)
 #undef ENC
 }
 
@@ -860,7 +928,7 @@ void psb_launch_update(cudaStream_t s, int kind, int wire, int opt, const Update
   }
   UPD(KIND_DENSE, WIRE_F32) UPD(KIND_DENSE, WIRE_BF16) UPD(KIND_DENSE, WIRE_F16) UPD(KIND_DENSE, WIRE_E4M3)
   UPD(KIND_DENSE, WIRE_E5M2) UPD(KIND_SCALED, WIRE_I8) UPD(KIND_SCALED, WIRE_E4M3) UPD(KIND_SCALED, WIRE_E5M2)
-  UPD(KIND_SCALED, WIRE_F16) UPD(KIND_TOPK, WIRE_F32) UPD(KIND_TOPK, WIRE_BF16)
+  UPD(KIND_SCALED, WIRE_F16) UPD(KIND_TOPK, WIRE_F32) UPD(KIND_TOPK, WIRE_BF16) UPD(KIND_QSGD, WIRE_I8)
 #undef UPD
 }
 

@@ -34,7 +34,7 @@ from typing import Dict, List, Optional
 import torch
 
 from .. import runtime
-from ..codings import KIND_DENSE, KIND_SCALED, KIND_TOPK, TILE, WIRE_BF16, WIRE_F16, WIRE_F32, wire_code_of
+from ..codings import KIND_DENSE, KIND_QSGD, KIND_SCALED, KIND_TOPK, TILE, WIRE_BF16, WIRE_F16, WIRE_F32, wire_code_of
 from ..ops import ext
 from ..utils.misc import CudaStepTimer
 from .layout import FlatLayout
@@ -252,6 +252,9 @@ class DeviceEngine:
         self._gates: list = []
         self._prof = CudaStepTimer(bool(getattr(opt, "profile", False)))
         self._epoch = 0                       # completed engine steps (the epoch-flag clock)
+        # block-wise QSGD: the step word of the Philox counter.  Counts every step of the run and is never rewound (recover()
+        # restarts the epoch clock, not this), so no (seed, rank, step) key repeats; checkpoints carry it (MPI_PS.state_dict)
+        self.rng_step = 0
         # async bookkeeping
         self.version = 0
         self._consumed = torch.zeros(64, dtype=torch.int64, device=self.device)
@@ -510,12 +513,15 @@ class DeviceEngine:
         items, self._chunk_items[k] = self._chunk_items[k], []
         if items:
             grads = [g for _, g in items]
+            qsgd = {}
+            if self.kind == KIND_QSGD:
+                qsgd = dict(levels=self.spec.levels, seed=self.spec.seed, rng_step=self.rng_step & 0xFFFFFFFF, rank=self.rank)
             m.encode(self.kind, self.wire, grads, [s.first_tile for s, _ in items],
                      [s.ntiles for s, _ in items], [s.index for s, _ in items],
                      self._tiles_ptr, self._wire_ptr, self._scales_ptr, self._amax_ptr, self._residual_ptr,
                      self.bpt, self.cap, self._ratio,
                      *((sig[0], sig[1], sig[2], self._sigctr_ptr) if sig else ([], 0, 0, 0)),
-                     csh)
+                     csh, **qsgd)
             nb = (len(items) + 63) // 64
             self.launches += nb * (2 if self.kind == KIND_SCALED else 1)
             self._keep.extend(grads)
@@ -712,6 +718,7 @@ class DeviceEngine:
         data["packaged_bytes"] = wire_bytes / nfired
         data["engine"] = "device"
         self._epoch += 1
+        self.rng_step += 1
         if len(self._fired) != L.nparams:
             self._uniform_steps = False              # some parameter sat this step out: per-parameter counts diverge from now on
         for i in self._fired:
@@ -758,7 +765,8 @@ class DeviceEngine:
         chunks; chunks gathered before the stall may already have been applied and published).  So: quiesce, clear every
         rank's signal pad and error slot, restart the epoch / chunk clocks at zero, re-adopt rank 0's parameters (and, in
         ``allgather`` mode where optimizer state is replicated, rank 0's state and step counts — through the slow object
-        path: this is a rare event), and re-open.  Optimizer step counts keep counting the failed step."""
+        path: this is a rare event), and re-open.  Optimizer step counts keep counting the failed step, and so does the QSGD
+        RNG step (a rounding draw is never reused)."""
         torch.cuda.synchronize(self.device)
         self.world.barrier()                  # every rank is here: nobody launches into the old epoch any more
         with torch.no_grad():

@@ -47,6 +47,7 @@ from .utils.misc import _bytes_of, find_param  # noqa: F401  (reference helpers,
 __all__ = ["MPI_PS", "SGD", "Adam", "_bytes_of", "find_param"]
 
 _MODES = ("ps", "allgather", "async")
+_QSGD_RNG_KEY = "qsgd_rng_step"      # extra top-level key of MPI_PS.state_dict() with a block-wise QSGD device engine
 _TAG_GRAD, _TAG_PARAM = 11, 12
 
 
@@ -206,7 +207,7 @@ class MPI_PS(torch.optim.Optimizer):
             ok = len(dts) == 1 and next(iter(dts)) in (torch.float32, torch.bfloat16, torch.float16)
         if engine == "device" and not ok:
             raise ValueError("engine='device' needs CUDA parameters of one float dtype and a built-in "
-                             "coding with a device_spec() (Identity / Cast / Scale / block-wise TopK)")
+                             "coding with a device_spec() (Identity / Cast / Scale / block-wise TopK / block-wise QSGD)")
         return ok
 
     def close(self):
@@ -585,9 +586,18 @@ class MPI_PS(torch.optim.Optimizer):
     def state_dict(self):
         if self._engine is not None:
             self._engine.sync_state_to_torch()
-        return super().state_dict()
+        sd = super().state_dict()
+        if self._engine is not None and self._engine.kind == _codings.KIND_QSGD:
+            # every rank's RNG step: a resumed run draws the same roundings as the uninterrupted one
+            sd[_QSGD_RNG_KEY] = self._engine.rng_step
+        return sd
 
     def load_state_dict(self, state_dict):
+        rng_step = state_dict.get(_QSGD_RNG_KEY)
+        if rng_step is not None:
+            state_dict = {k: v for k, v in state_dict.items() if k != _QSGD_RNG_KEY}
+            if self._engine is not None and self._engine.kind == _codings.KIND_QSGD:
+                self._engine.rng_step = int(rng_step)
         super().load_state_dict(state_dict)
         if self._engine is not None:
             # torch casts loaded state to the parameter dtype (bf16); the engine's state is fp32, so hand
