@@ -535,8 +535,11 @@ std::vector<at::Tensor> stem_fwd(const at::Tensor& x, const at::Tensor& w2d, boo
   TORCH_CHECK(W % 8 == 0 && W <= 256 && W >= 8, "fused stem: W must be a multiple of 8 and <= 256");
   auto a = im2col_stem(x);                                           // the REAL (emulated) patch-matrix kernel
   auto y32 = at::matmul(a.to(at::kFloat), w2d.to(at::kFloat).t());   // [M,64], fp32 accumulators
-  at::Tensor sums = want_sums ? at::cat({y32.sum(0), (y32 * y32).sum(0)}).contiguous() : at::Tensor();
-  return {y32.to(at::kBFloat16).view({N, OH, OW, 64}).permute({0, 3, 1, 2}), sums};
+  auto y = y32.to(at::kBFloat16);
+  // like the kernel's epilogue: the sums are taken over the bf16 values it stores, not over the fp32 accumulators
+  auto yr = y.to(at::kFloat);
+  at::Tensor sums = want_sums ? at::cat({yr.sum(0), (yr * yr).sum(0)}).contiguous() : at::Tensor();
+  return {y.view({N, OH, OW, 64}).permute({0, 3, 1, 2}), sums};
 }
 
 at::Tensor stem_wgrad(const at::Tensor& x, const at::Tensor& gy) {
